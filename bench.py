@@ -27,6 +27,13 @@ Keys beyond the base contract:
 --impl reference times the reference's own CPU implementation with every host thread it
 can use (as many concurrent encoder instances as fit; one instance = 1 + nthreads
 pthreads) and prints the same JSON line with "impl": "reference".
+
+--dump-outputs DIR writes what the last timed step computed, as float32 arrays of whole
+lines of int16 IQ (I, Q interleaved; rows in stream order): DIR/iq.npy from the
+device-resident step, a fixed seeded choice of lines of each of its render calls, gathered on
+the device after each call of that step; DIR/e2e_iq.npy a seeded choice of lines of the host
+buffer of the last end-to-end step. 60 MB at most in all. The inputs (test pattern and tone) are the
+same on every run, so two builds run with the same arguments can be compared array for array.
 """
 import argparse
 import json
@@ -35,6 +42,8 @@ import subprocess
 import sys
 import threading
 import time
+
+import numpy as np
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
@@ -53,6 +62,19 @@ REF_THREADS = 3          # main/raster + vfilter + audio (reference video.c:4692
 NCU = {"file": "profiles/r02_ncu_k_line_raw.txt", "lines": 40000, "dram_read": 47_632_128, "dram_write": 113_646_080,
        "warp_instructions": 238_153_871, "issue_active_pct": 61.8}
 KERNEL = "k_line (fused line kernel: raster + chroma and video filters on the tensor cores + sound carriers + IQ store)"
+DUMP_BYTES = {"iq": 45_000_000, "e2e_iq": 15_000_000}     # --dump-outputs: float32 bytes per array
+
+
+def dump_lines(lines, calls, values_per_line, nbytes):
+    """--dump-outputs: for each of `calls` render calls of `lines` lines, a sorted choice of its lines, as many
+    as fit `nbytes` of float32 over all calls; seeded, so the same on every run."""
+    k = max(1, min(lines, nbytes // 4 // values_per_line // calls))
+    rng = np.random.default_rng(0)
+    return np.stack([np.sort(rng.choice(lines, k, replace=False)) for _ in range(calls)])
+
+
+def save_dump(directory, name, rows):
+    np.save(os.path.join(directory, name + ".npy"), rows.reshape(-1, rows.shape[-1]).astype(np.float32))
 
 
 def measured_peak_gbs():
@@ -386,7 +408,10 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-e2e", action="store_true")
     ap.add_argument("--no-extra", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write what the last timed step computed to DIR/*.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
 
     rank = int(os.environ.get("RANK", "0"))
     local = int(os.environ.get("LOCAL_RANK", "0"))
@@ -396,7 +421,6 @@ def main():
         bench_reference(args, rank, world)
         return
 
-    import numpy as np
     import torch
     import torch.distributed as dist
     import hacktv_b200 as H
@@ -423,14 +447,24 @@ def main():
     # ---- device-resident throughput ("value") ---------------------------------
     enc, out, chunk, calls, nsamp, l0, ev0, ev1 = device_resident(H, torch, mode, rate, filt, args.frames, args.steps, args.warmup, stream)
     nlines = chunk * calls
+    dump = args.dump_outputs if rank == 0 else None
+    picked = None
+    if dump:
+        os.makedirs(dump, exist_ok=True)
+        out_lines = out.view(chunk, -1)
+        pick = torch.from_numpy(dump_lines(chunk, calls, out_lines.shape[1], DUMP_BYTES["iq"])).cuda()
+        picked = torch.empty((calls, pick.shape[1], out_lines.shape[1]), dtype=torch.int16, device="cuda")
+        torch.index_select(out_lines, 0, pick[0], out=picked[0])       # its first launch loads the kernel: not timed
     barrier()
     with ClockSampler(local) as clk:
         time.sleep(0.005)
         clk.t0 = time.perf_counter()
         ev0.record()
-        for _ in range(args.steps):
-            for _ in range(calls):
+        for step in range(args.steps):
+            for c in range(calls):
                 enc.render(chunk, out.data_ptr(), stream)
+                if picked is not None and step == args.steps - 1:      # the next call overwrites `out`
+                    torch.index_select(out_lines, 0, pick[c], out=picked[c])
         ev1.record()
         barrier()
         clk.t1 = time.perf_counter()
@@ -445,6 +479,8 @@ def main():
         kern_ms.append(enc.last_line_kernel_ms())
     kern_lines = enc.last_line_kernel_lines()
     checksum = int(out[:4096].to(torch.int32).sum().item())
+    if picked is not None:
+        save_dump(dump, "iq", picked.cpu().numpy())
     width = enc.width
     enc.close()
     del out
@@ -470,6 +506,10 @@ def main():
             enc2.render_host_ptr(e2e_lines, host.data_ptr())
         torch.cuda.synchronize()
         dt = time.perf_counter() - t0
+        if dump:
+            per = 2 if enc2.complex else 1
+            rows = host[: e2e_lines * enc2.width * per].view(e2e_lines, -1).numpy()
+            save_dump(dump, "e2e_iq", rows[dump_lines(e2e_lines, 1, rows.shape[1], DUMP_BYTES["e2e_iq"])])
         e2e_samples = e2e_lines * enc2.width
         e2e_s, e2e_job = reduce_job(torch, dist, world, dt, e2e_samples * args.steps)
         h2d = e2e_frames * enc2.active_width * enc2.active_lines * 4 + int(e2e_samples / rate * 32000) * 4

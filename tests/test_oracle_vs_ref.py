@@ -1,12 +1,78 @@
-"""The oracle against the reference itself (oracle/_ref/ref_harness, the unmodified
-fsphil/hacktv sources compiled in place): bit-exact, incl. inputs and options the golden
-fixtures do not cover. Skipped where the prebuilt reference is absent."""
+"""The oracle against the reference itself (the unmodified fsphil/hacktv sources, run through
+oracle/ref_harness.c): bit-exact, incl. inputs and options the golden fixtures of
+test_oracle_golden.py do not cover. What the reference emitted is stored in tests/golden/vs_ref.json
+(sha256 and size of every stream) and tests/golden/vs_ref.npz (an evenly spaced sample of each;
+short streams, such as the WSS lines taken apart below, whole). tests/golden/make_golden_vs_ref.py
+makes both by running these tests against the reference binaries built by `make -C oracle ref`."""
+import hashlib
+import json
+import os
+
 import numpy as np
 import pytest
 
 import orc
 
-pytestmark = pytest.mark.skipif(not orc.have_ref(), reason="oracle/_ref not built (needs /root/reference at build time)")
+HERE = os.path.dirname(os.path.abspath(__file__))
+GOLD_JSON = os.path.join(HERE, "golden", "vs_ref.json")
+GOLD_NPZ = os.path.join(HERE, "golden", "vs_ref.npz")
+SAMPLE = 2048           # values of each stream kept: they say which values differ when the digest does
+
+# tests/golden/make_golden_vs_ref.py sets this to a dict: the comparisons below then run the reference
+# binaries, check against their output and record it under each key
+RECORD = None
+_gold = None
+
+
+def _key(*parts):
+    return " ".join(str(p) for p in parts)
+
+
+def _digest(a):
+    a = np.ascontiguousarray(a)
+    stride = -(-a.size // SAMPLE)
+    return {"sha256": hashlib.sha256(a.tobytes()).hexdigest(), "size": int(a.size), "sample": a.ravel()[::stride].copy()}
+
+
+def _stored(key):
+    global _gold
+    if _gold is None:
+        with open(GOLD_JSON) as f:
+            meta = json.load(f)
+        z = np.load(GOLD_NPZ)
+        _gold = {k: dict(v, sample=z[k]) for k, v in meta.items()}
+    return _gold[key]
+
+
+def _reference(key, args, kw, view):
+    want = orc.run_ref(*args, **kw)
+    if view is not None:
+        want = view(want)
+    RECORD[key] = _digest(want)
+    return want
+
+
+def assert_reference(got, key, *args, view=None, **kw):
+    """got equals what orc.run_ref(*args, **kw) emits (through `view`), stored under `key`."""
+    if RECORD is not None:
+        want = _reference(key, args, kw, view)
+        assert np.array_equal(got, want), f"{key}: {np.count_nonzero(got != want)} values differ"
+        return
+    g, d = _stored(key), _digest(got)
+    assert d["size"] == g["size"], f"{key}: {d['size']} values, the reference emitted {g['size']}"
+    bad = np.count_nonzero(d["sample"] != g["sample"])
+    assert bad == 0, f"{key}: {bad} of {g['sample'].size} sampled values differ"
+    assert d["sha256"] == g["sha256"], f"{key}: the sampled values agree, others differ"
+
+
+def reference_values(key, *args, view=None, **kw):
+    """What orc.run_ref(*args, **kw) emits (through `view`): short streams, stored whole under `key`."""
+    if RECORD is not None:
+        return _reference(key, args, kw, view)
+    g = _stored(key)
+    assert g["sample"].size == g["size"], f"{key} is not stored whole"
+    return g["sample"]
+
 
 CASES = [
     ("pal", 16000000, 700, False, ()),
@@ -56,9 +122,7 @@ def test_oracle_equals_reference(built, mode, rate, nlines, filt, extra):
     o.open_test_source()
     got = o.render(nlines)
     o.close()
-    want = orc.run_ref(mode, rate, nlines, vfilter=filt, extra=extra)
-    assert got.size == want.size
-    assert np.array_equal(got, want), f"{np.count_nonzero(got != want)} values differ"
+    assert_reference(got, _key("test", mode, rate, nlines, filt, *extra), mode, rate, nlines, vfilter=filt, extra=extra)
 
 
 PASSTHRU_CASES = [
@@ -84,10 +148,14 @@ def test_passthru_alignment(built, tmp_path, mode, rate, filt, extra, ext_lines)
     o.close()
     fn = tmp_path / "ext.iq"
     ext.tofile(fn)
-    want = orc.run_ref(mode, rate, 30, vfilter=filt, extra=tuple(extra) + ("--passthru", str(fn)))
-    assert np.array_equal(got, want), f"{np.count_nonzero(got != want)} values differ"
-    plain = orc.run_ref(mode, rate, 30, vfilter=filt, extra=extra)
-    assert not np.array_equal(plain, want)
+    assert_reference(got, _key("passthru", mode, rate, filt, ext_lines, *extra), mode, rate, 30, vfilter=filt,
+                     extra=tuple(extra) + ("--passthru", str(fn)))
+    o = orc.Oracle(_conf(built, mode, filt, extra), rate)
+    o.open_test_source()
+    plain = o.render(30)
+    o.close()
+    assert_reference(plain, _key("plain", mode, rate, 30, filt, *extra), mode, rate, 30, vfilter=filt, extra=extra)
+    assert not np.array_equal(plain, got)
 
 
 def wss_overlay(built, mode, rate, wss="16:9"):
@@ -100,8 +168,13 @@ def wss_overlay(built, mode, rate, wss="16:9"):
     black = int(t.get("levels")[1])
     t.close()
     per = 2 if conf.output_type == 0 else 1
-    plain = orc.run_ref(mode, rate, 30, extra=("--noaudio", "--nocolour")).reshape(30, W, per)[22, :, 0].astype(np.int32)
-    with_wss = orc.run_ref(mode, rate, 30, extra=("--noaudio", "--nocolour", "--wss", wss)).reshape(30, W, per)[22, :, 0].astype(np.int32)
+
+    def line23(x):
+        return x.reshape(30, W, per)[22, :, 0]
+    plain = reference_values(_key("line23", mode, rate), mode, rate, 30, extra=("--noaudio", "--nocolour"),
+                             view=line23).astype(np.int32)
+    with_wss = reference_values(_key("line23 wss", mode, rate, wss), mode, rate, 30,
+                                extra=("--noaudio", "--nocolour", "--wss", wss), view=line23).astype(np.int32)
     blank_to = int(round(rate * 42.5e-6))
     base = plain.copy()
     base[half:blank_to] = black
@@ -120,8 +193,8 @@ def test_vbi_overlay_is_where_the_reference_puts_wss(built, mode, rate, filt, ex
     o.add_vbi_line(23, add, rep)
     got = o.render(700)
     o.close()
-    want = orc.run_ref(mode, rate, 700, vfilter=filt, extra=tuple(extra) + ("--wss", "16:9"))
-    assert np.array_equal(got, want), f"{np.count_nonzero(got != want)} values differ"
+    assert_reference(got, _key("wss", mode, rate, 700, filt, *extra), mode, rate, 700, vfilter=filt,
+                     extra=tuple(extra) + ("--wss", "16:9"))
 
 
 def test_oracle_equals_reference_on_random_input(built):
@@ -133,16 +206,22 @@ def test_oracle_equals_reference_on_random_input(built):
     o.set_source(frames, audio)
     got = o.render(1400)
     o.close()
-    want = orc.run_ref("i", 16000000, 1400, vfilter=True, frames=frames, audio=audio, audio_block=4000)
-    assert np.array_equal(got, want)
+    assert_reference(got, "random i 16000000 1400", "i", 16000000, 1400, vfilter=True, frames=frames, audio=audio,
+                     audio_block=4000)
 
 
-def test_unpatched_heap_differs_only_near_line_ends():
+def test_unpatched_heap_differs_only_near_line_ends(built):
     """The stock allocator lets the chroma FIR read past its buffer (SURVEY.md §8c): the
-    masked comparison - everything further than 32 samples from a line boundary - is exact."""
-    a = orc.run_ref("i", 16000000, 700, vfilter=True).reshape(700, 1024, 2)
-    b = orc.run_ref("i", 16000000, 700, vfilter=True, rawheap=True).reshape(700, 1024, 2)
-    assert np.array_equal(a[:, 32:-32], b[:, 32:-32])
+    masked comparison - everything further than 32 samples from a line boundary - is exact
+    (against the oracle, which equals the zero-heap build everywhere: test_oracle_equals_reference)."""
+    def masked(x):
+        return x.reshape(700, 1024, 2)[:, 32:-32]
+    o = orc.Oracle(built.mode_config("i", vfilter=True), 16000000)
+    o.open_test_source()
+    got = masked(o.render(700))
+    o.close()
+    assert_reference(got, "rawheap masked i 16000000 700 True", "i", 16000000, 700, vfilter=True, rawheap=True,
+                     view=masked)
 
 
 # --pixelrate (SURVEY.md section 8f rank 4): raster at the pixel rate, the reference's polyphase resampler
@@ -170,9 +249,8 @@ def test_pixelrate_resampler_equals_reference(built, mode, rate, prate, nlines, 
     o.open_test_source()
     got = o.render(nlines)
     o.close()
-    want = orc.run_ref(mode, rate, nlines, vfilter=filt, extra=tuple(extra) + ("--pixelrate", str(prate)))
-    assert got.size == want.size
-    assert np.array_equal(got, want), f"{np.count_nonzero(got != want)} values differ"
+    assert_reference(got, _key("pixelrate", mode, rate, prate, nlines, filt, *extra), mode, rate, nlines, vfilter=filt,
+                     extra=tuple(extra) + ("--pixelrate", str(prate)))
 
 
 def test_pixelrate_later_window_and_random_input(built):
@@ -182,8 +260,8 @@ def test_pixelrate_later_window_and_random_input(built):
     o.open_test_source()
     got = o.render(1700)[1400 * 2048:]
     o.close()
-    want = orc.run_ref("i", 16000000, 300, skip=1400, vfilter=True, extra=("--pixelrate", "13500000"))
-    assert np.array_equal(got, want)
+    assert_reference(got, "pixelrate skip 1400 i 16000000 13500000 300 True", "i", 16000000, 300, skip=1400,
+                     vfilter=True, extra=("--pixelrate", "13500000"))
     rng = np.random.default_rng(5)
     o = orc.Oracle(conf, 16000000, 13500000)
     frames = rng.integers(0, 1 << 24, size=(2, o.active_lines, o.active_width), dtype=np.uint32)
@@ -191,9 +269,8 @@ def test_pixelrate_later_window_and_random_input(built):
     o.set_source(frames, audio)
     got = o.render(900)
     o.close()
-    want = orc.run_ref("i", 16000000, 900, vfilter=True, frames=frames, audio=audio, audio_block=4000,
-                       extra=("--pixelrate", "13500000"))
-    assert np.array_equal(got, want)
+    assert_reference(got, "pixelrate random i 16000000 13500000 900 True", "i", 16000000, 900, vfilter=True,
+                     frames=frames, audio=audio, audio_block=4000, extra=("--pixelrate", "13500000"))
 
 
 def test_pixelrate_with_passthru_and_wss(built, tmp_path):
@@ -209,8 +286,8 @@ def test_pixelrate_with_passthru_and_wss(built, tmp_path):
     o.close()
     fn = tmp_path / "ext.iq"
     ext.tofile(fn)
-    want = orc.run_ref("i", 16000000, 30, vfilter=True, extra=("--pixelrate", "13500000", "--passthru", str(fn)))
-    assert np.array_equal(got, want), f"{np.count_nonzero(got != want)} values differ"
+    assert_reference(got, "pixelrate passthru i 16000000 13500000 30 True", "i", 16000000, 30, vfilter=True,
+                     extra=("--pixelrate", "13500000", "--passthru", str(fn)))
 
     add, rep = wss_overlay(built, "pal", 13500000)               # the waveform at the pixel rate
     o = orc.Oracle(built.mode_config("pal"), 16000000, 13500000)
@@ -218,8 +295,8 @@ def test_pixelrate_with_passthru_and_wss(built, tmp_path):
     o.add_vbi_line(23, add, rep)
     got = o.render(100)
     o.close()
-    want = orc.run_ref("pal", 16000000, 100, extra=("--pixelrate", "13500000", "--wss", "16:9"))
-    assert np.array_equal(got, want), f"{np.count_nonzero(got != want)} values differ"
+    assert_reference(got, "pixelrate wss pal 16000000 13500000 100 False", "pal", 16000000, 100,
+                     extra=("--pixelrate", "13500000", "--wss", "16:9"))
 
 
 def test_pixelrate_pairs_the_oracle_does_not_restate(built):
